@@ -23,6 +23,9 @@ iterations-executed honours the reference's early return, lib/bundle_entropy.py:
 
 --impl reference: times the CPU implementation only (oracle port; the reference itself is Python and
 /root/reference does not exist on the GPU box), all host cores, same metric/config; loads no native code.
+
+--dump-outputs DIR: after the timed steps of the headline workload, write what its last step returned (y*, the
+bundle, nIters; see dump_outputs) as DIR/<name>.npy, so that two builds can be compared output for output.
 """
 import argparse
 import json
@@ -313,7 +316,41 @@ def measure_fp64_peak(ctx):
     return best
 
 
-def measure_workload(ctx, name, steps, warmup, scaling, solver, cpu_seconds, headline):
+DUMP_X_BYTES = 32 << 20         # --dump-outputs: y* rows and their per-row scalars
+DUMP_BUNDLE_BYTES = 24 << 20    # --dump-outputs: bundle rows (A in float32 + xs in float64, KS x n each; b, lam)
+
+
+def dump_outputs(out_dir, st):
+    """Write what solveBatch returns, (x, A, b, lam, xs, nIters), for a fixed sample of rows of ``st`` as
+    out_dir/<name>.npy: x [R, n] and nIters / counts [R] for R rows (all rows when they fit DUMP_X_BYTES, else a
+    sample drawn with a fixed seed), A / xs [R', KS, n] and b / lam [R', KS] for R' of those rows spread evenly
+    (DUMP_BUNDLE_BYTES), in bundle order (A[u][j] = the reference's ragged A[u][j]), zero past counts; row_index /
+    bundle_row_index give the rows.  Every array is float32 or float64; the sample depends only on the shape."""
+    import torch
+    B, n, KS = st.B, st.n, st.KS
+    nx = min(B, max(1, DUMP_X_BYTES // (8 * n + 3 * 8)))                   # x, nIters, counts, row_index
+    nb = min(nx, max(1, DUMP_BUNDLE_BYTES // (KS * (12 * n + 16) + 8)))    # A, xs, b, lam, bundle_row_index
+    rows = np.arange(B) if nx == B else np.sort(np.random.RandomState(0).choice(B, nx, replace=False))
+    brows = rows[np.linspace(0, nx - 1, nb).round().astype(np.int64)]
+    out = {"row_index": rows.astype(np.float64), "bundle_row_index": brows.astype(np.float64)}
+    idx = torch.from_numpy(rows).to(st.y.device)
+    out["x"] = st.y.index_select(0, idx).cpu().numpy()
+    out["nIters"] = st.nIters.index_select(0, idx).cpu().numpy().astype(np.float64)
+    out["counts"] = st.count.index_select(0, idx).cpu().numpy().astype(np.float64)
+    bidx = torch.from_numpy(brows).to(st.y.device)
+    perm = st.perm.index_select(0, bidx).long().clamp_(0, KS - 1)
+    live = torch.arange(KS, device=perm.device)[None, :] < st.count.index_select(0, bidx)[:, None]
+    for name, src in (("b", st.h), ("lam", st.lam)):
+        out[name] = (src.index_select(0, bidx).gather(1, perm) * live).cpu().numpy()
+    for name, src in (("A", st.G), ("xs", st.ys)):
+        v = src.index_select(0, bidx).gather(1, perm[:, :, None].expand(-1, -1, n))
+        out[name] = (v * live[:, :, None]).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure_workload(ctx, name, steps, warmup, scaling, solver, cpu_seconds, headline, dump_dir=None):
     """value / e2e / per-kernel roofline / cpu_baseline of one workload on this rank set."""
     import ctypes as C
     import torch
@@ -400,6 +437,8 @@ def measure_workload(ctx, name, steps, warmup, scaling, solver, cpu_seconds, hea
     t_wall = time.perf_counter() - t_wall0
     if clk:
         clk.__exit__()
+    if dump_dir and rank == 0:      # before the passes below overwrite the state
+        dump_outputs(dump_dir, st)
     ms_per_step = allmax(sum(a.elapsed_time(b) for a, b in ev)) / steps
     value = Bglob * its / (ms_per_step * 1e-3)
 
@@ -651,7 +690,8 @@ def run_gpu(args):
     ctx.fp64_peak = measure_fp64_peak(ctx)
     scaling = args.scaling or "strong"
     cpu_s = 0.0 if args.no_cpu_baseline else args.cpu_seconds
-    head = measure_workload(ctx, args.workload, args.steps, max(3, args.warmup), scaling, args.solver, cpu_s, True)
+    head = measure_workload(ctx, args.workload, args.steps, max(3, args.warmup), scaling, args.solver, cpu_s, True,
+                            args.dump_outputs)
     subs = {}
     if ctx.world == 1 and not args.no_sub:
         for w in SUB_WORKLOADS:
@@ -729,6 +769,10 @@ def run_reference(args):
 
 
 def main():
+    # the benchmark writes nothing into the tree it runs from (which may be read-only): no __pycache__ beside the
+    # sources, here or in the CPU arm's worker processes (they inherit the environment)
+    sys.dont_write_bytecode = True
+    os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=5)
@@ -744,7 +788,13 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     ap.add_argument("--sub-cpu-seconds", type=float, default=6.0)
     ap.add_argument("--sub-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline workload's outputs of the last timed step (rank 0's rows) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.sub_steps < 1:
+        ap.error("--steps and --sub-steps must be >= 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm has none to write")
     args.no_sub = args.no_sub or args.no_target_shape
     try:
         if args.impl == "reference":

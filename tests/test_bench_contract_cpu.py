@@ -73,14 +73,59 @@ def test_reference_arm_under_torchrun_prints_one_line_from_rank_0():
     assert d["impl"] == "reference" and d["n_gpus"] == 2 and d["value"] > 0 and d["native_modules_loaded"] == []
 
 
-def test_algorithmic_work_models_match_survey_8d():
-    """The roofline numerators: FLOP_fg = 4 * MAC per solve (SURVEY.md 8d: C2 9.45 M, C3 0.866 M, C4 0.170 M,
-    C5 79.7 M, T 8.39 M) and the K2 FP64 model n (k^2 + 11 k + 30) per interior-point iteration (DESIGN.md section 3)."""
+def _load_bench():
     import importlib.util
-    import numpy as np
     spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_dump_outputs_writes_the_ragged_results_of_sampled_rows(tmp_path, monkeypatch):
+    """--dump-outputs: the arrays solveBatch returns for a fixed row sample, bundle rows in perm order (what the
+    ragged A / b / lam / xs views hold), zero past counts, float32 / float64 only, within the 64 MB budget."""
+    import types
+    import numpy as np
+    bench = _load_bench()
+    assert bench.DUMP_X_BYTES + bench.DUMP_BUNDLE_BYTES + 16 * 1024 <= 64 << 20
+    B, n, KS = 9, 5, 4
+    g = torch.Generator().manual_seed(0)
+    st = types.SimpleNamespace(
+        B=B, n=n, KS=KS, y=torch.rand(B, n, generator=g, dtype=torch.float64),
+        G=torch.randn(B, KS, n, generator=g), ys=torch.rand(B, KS, n, generator=g, dtype=torch.float64),
+        h=torch.randn(B, KS, generator=g, dtype=torch.float64), lam=torch.rand(B, KS, generator=g, dtype=torch.float64),
+        perm=torch.stack([torch.randperm(KS, generator=g) for _ in range(B)]).int(),
+        count=torch.randint(0, KS + 1, (B,), generator=g).int(), nIters=torch.randint(1, 6, (B,), generator=g).int())
+    monkeypatch.setattr(bench, "DUMP_X_BYTES", 6 * (8 * n + 24))                # 6 of 9 rows
+    monkeypatch.setattr(bench, "DUMP_BUNDLE_BYTES", 4 * (KS * (12 * n + 16) + 8))  # 4 of those 6
+    runs = []
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), st)
+        runs.append({f[:-4]: np.load(str(tmp_path / d / f)) for f in os.listdir(str(tmp_path / d))})
+    out = runs[0]
+    assert sorted(out) == ["A", "b", "bundle_row_index", "counts", "lam", "nIters", "row_index", "x", "xs"]
+    for k, a in out.items():
+        assert a.dtype in (np.float32, np.float64), k
+        np.testing.assert_array_equal(a, runs[1][k], err_msg=k)       # same state -> same sample, same files
+    rows, brows = out["row_index"].astype(int), out["bundle_row_index"].astype(int)
+    assert len(rows) == 6 and len(set(rows)) == 6 and len(brows) == 4 and set(brows) <= set(rows)
+    np.testing.assert_array_equal(out["x"], st.y.numpy()[rows])
+    np.testing.assert_array_equal(out["nIters"], st.nIters.numpy()[rows])
+    np.testing.assert_array_equal(out["counts"], st.count.numpy()[rows])
+    assert out["A"].dtype == np.float32 and out["A"].shape == (4, KS, n) and out["xs"].shape == (4, KS, n)
+    for i, u in enumerate(brows):
+        k = int(st.count[u])
+        slots = st.perm.numpy()[u, :k]
+        for name, src in (("A", st.G), ("xs", st.ys), ("b", st.h), ("lam", st.lam)):
+            np.testing.assert_array_equal(out[name][i, :k], src.numpy()[u, slots], err_msg=name)
+            assert not np.any(out[name][i, k:]), name
+
+
+def test_algorithmic_work_models_match_survey_8d():
+    """The roofline numerators: FLOP_fg = 4 * MAC per solve (SURVEY.md 8d: C2 9.45 M, C3 0.866 M, C4 0.170 M,
+    C5 79.7 M, T 8.39 M) and the K2 FP64 model n (k^2 + 11 k + 30) per interior-point iteration (DESIGN.md section 3)."""
+    import numpy as np
+    bench = _load_bench()
     from icnn_b200 import workloads
     want = {"C1": 4 * 536, "C2": 4 * 2361856, "C3": 4 * 216399, "C4": 4 * 42606, "C5": 4 * 19928064, "T": 4 * 2098688}
     for name, flops in want.items():
